@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (sm_100a kernels)
     python bench.py --impl reference --gpus N --steps K ...   # CPU restatement of the PyG path
+    python bench.py ... --dump-outputs DIR                    # + the last timed step's results as DIR/<name>.npy
 
 Workload at N=1 (BASELINE.json configs[2], the configuration the metric is quoted on): the SGCN
 network of util/networks.py with the GCNConv branch (13 conv blocks, widths
@@ -68,7 +69,16 @@ def parse():
     ap.add_argument("--mode", default="replicas", choices=["replicas", "partition"],
                     help="replicas: one independent mesh per GPU (default, configs[2]/[4]); partition: ONE mesh vertex-partitioned over the "
                          "GPUs with per-propagation halo exchange over NCCL (configs[3], strong scaling)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed train step computed (network output, loss, parameters and "
+                         "buffers after the optimizer step, parameter gradients) as DIR/<name>.npy, rank 0's mesh; the inputs are "
+                         "seeded, so two builds run with the same arguments can be compared array by array (bench_outputs/ is git-ignored)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.mode != "replicas"):
+        ap.error("--dump-outputs covers the train step of the GPU arm in replicas mode")
+    return args
 
 
 # ------------------------------------------------------------------------------------------
@@ -203,6 +213,35 @@ def gcnconv_layer_bench(edge_index, n: int, nnz: int, dev, pk, cin: int = 256, c
             "hbm_frac": gbs / pk["hbm_gbs"], "reps": reps}
 
 
+DUMP_MAX_BYTES = 60 << 20       # array bytes; with the .npy headers the files stay under 64 MB (10^6 bytes each)
+
+
+def dump_outputs(path: str, net, loss, out) -> None:
+    """``--dump-outputs``: the train step's results as float32 / float64 .npy files.  The output rows are capped so that
+    the files stay under 64 MB in all: above the cap a fixed, seeded sample of rows (sorted) is written, the same for every
+    run with the same arguments."""
+    import numpy as np
+    arrays = {"loss": loss}
+    for k, v in net.state_dict().items():
+        if v.is_floating_point():
+            arrays[f"state.{k}"] = v
+    for k, p in net.named_parameters():
+        if p.grad is not None:
+            arrays[f"grad.{k}"] = p.grad
+    arrays = {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+    room = DUMP_MAX_BYTES - sum(a.nbytes for a in arrays.values())
+    out = out.detach()
+    row_bytes = out.shape[1] * out.element_size()
+    if out.shape[0] * row_bytes > room:
+        rows = torch.randperm(out.shape[0], generator=torch.Generator().manual_seed(0))[:room // row_bytes].sort()[0]
+        out = out[rows.to(out.device)]
+    arrays["output"] = out.cpu().numpy()
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (k, a.dtype)
+        np.save(os.path.join(path, f"{k}.npy"), a)
+
+
 def make_problem(freq: int, device, seed: int = 314, order: str = "given"):
     from semigcn_b200 import meshgen
     mesh = meshgen.icosphere(freq, device=device, dtype=torch.float64)
@@ -253,15 +292,16 @@ def run_ours(args, rank, world, local_rank):
                                    prob["dms"][:, 0:1].contiguous())
 
     def one_step(i, data_in, dm):
+        """One train step; returns (loss, network output)."""
         if graphed is not None:      # inputs (device or pinned host) are copied into the graph's static buffers, then one replay
-            return graphed(dm, None if data_in is data else data_in.z1, None if data_in is data else data_in.x_pos)
+            return graphed(dm, None if data_in is data else data_in.z1, None if data_in is data else data_in.x_pos), graphed.out
         opt.zero_grad(set_to_none=True)
         out = net(data_in, dm)
         loss = step_losses(out, prob)
         loss.backward()
         with profile.region("adam"):         # no-op unless the roofline pass below is active
             opt.step()
-        return loss
+        return loss, out
 
     def barrier():
         if world > 1:
@@ -279,12 +319,15 @@ def run_ours(args, rank, world, local_rank):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(args.steps):
-        one_step(i, data, prob["dms"][:, i % 8:i % 8 + 1])
+        loss, out = one_step(i, data, prob["dms"][:, i % 8:i % 8 + 1])
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
     launches = _lib.LAUNCHES - launches0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:      # before the passes below train the network further
+        dump_outputs(args.dump_outputs, net, loss, out)
+    del loss, out                            # the passes below run without the last step's output held
 
     # ---------------- per-kernel-family roofline pass (CUDA events on the launching stream)
     fam = {}
@@ -314,13 +357,13 @@ def run_ours(args, rank, world, local_rank):
 
     def e2e_step(i, last=False):
         if graphed is not None:      # graph mode: the mesh (edge_index) is fixed at capture; z1 / x_pos / mask come from pinned host memory
-            loss = one_step(i, Data(z1=h["z1"], x_pos=h["x_pos"], edge_index=None), h["dms"][i % 8])
+            loss, _ = one_step(i, Data(z1=h["z1"], x_pos=h["x_pos"], edge_index=None), h["dms"][i % 8])
             loss_host.copy_(loss.detach(), non_blocking=True)
             return
         if not last:
             submit(i + 1)
         d = pipe.get()
-        loss = one_step(i, Data(z1=d["z1"], x_pos=d["x_pos"], edge_index=d["edge_index"]), d["dm"])
+        loss, _ = one_step(i, Data(z1=d["z1"], x_pos=d["x_pos"], edge_index=d["edge_index"]), d["dm"])
         pipe.release()
         loss_host.copy_(loss.detach(), non_blocking=True)
 

@@ -188,9 +188,12 @@ def test_sgcn_oracle_runs_and_backprops():
 @pytest.mark.parametrize("conv", ["chebconv", "gcnconv"])
 @pytest.mark.parametrize("skip", [False, True])
 def test_oracle_sgcn_matches_reference_networks_py(conv, skip):
-    """tests/golden/ref_sgcn_n4.npz was produced by running /root/reference/util/networks.py::SingleScaleGCN itself
+    """tests/golden/ref_sgcn_n4.npz was produced by running the reference's util/networks.py::SingleScaleGCN itself
     (PyG symbols resolved to the oracle classes, tests/golden/make_golden_net.py): the oracle's restated network must
-    consume the RNG identically (same seeded initial state_dict) and give the same forward in train and eval mode."""
+    consume the RNG identically (same seeded initial state_dict, exactly) and give the same forward in train and eval mode.
+    The forward is held to REL_TOL, not to bit equality: the fixture's fp32 values depend on the host that computed them
+    (MKL's GEMM rounds differently by instruction set and thread count: up to 4.4e-6 norm-relative in train mode,
+    measured), while a wiring or RNG-order difference is O(1)."""
     import numpy as np
     gold = load_golden("ref_sgcn_n4.npz")
     tag = f"{conv}_{'skip' if skip else 'noskip'}"
@@ -205,10 +208,10 @@ def test_oracle_sgcn_matches_reference_networks_py(conv, skip):
     ei, dm = torch.from_numpy(gold["edge_index"]), torch.from_numpy(gold["dm"])
     net.train()
     y = net(z1, x_pos, ei, dm)
-    assert torch.equal(y.detach(), torch.from_numpy(gold[f"{tag}_train"]))
+    assert_close(y, torch.from_numpy(gold[f"{tag}_train"]), what="train-mode forward")
     net.eval()
     y = net(z1, x_pos, ei, dm)
-    assert torch.equal(y.detach(), torch.from_numpy(gold[f"{tag}_eval"]))
+    assert_close(y, torch.from_numpy(gold[f"{tag}_eval"]), what="eval-mode forward")
 
 
 @pytest.mark.parametrize("n", [4, 8])
