@@ -105,8 +105,8 @@ SGB_API int sgb_graph_build(const int64_t* edge_index, int64_t nnz, int64_t n, i
  *    laid out [sgb_spmm_stat_rows(n, c)][3][c]; feeds sgb_bn_finalize (Chan merge).
  *    Replaces MessagePassing.propagate (index_select -> mul -> scatter_add), fwd and,
  *    called with the transpose CSR, bwd.
- *    amax_out (optional, device float zeroed by the caller) receives max |Y| (atomicMax on the float
- *    bits): the scale of the fp16-split GEMM engine that consumes Y (sgb_gemm a_amax), for free.
+ *    amax_out (optional, device float zeroed by the caller) receives max |Y| over the finite entries
+ *    (atomicMax on the float bits): the scale of the fp16-split GEMM engine that consumes Y (sgb_gemm a_amax), for free.
  *    SGB_MODE_ADJ takes any CSR whose packed stream carries its own weights -- also a RECTANGULAR one
  *    (n = rows of Y; column ids index rows of X, which may have any row count > max column id; dis is
  *    not read): this is how MeshPool / MeshUnpool (reference util/meshnet.py:9-27, torch.sparse.mm of
@@ -158,8 +158,12 @@ SGB_API int sgb_gather_rows(const float* x, int64_t ldx, const int32_t* idx, int
  *    3 = tcgen05 2xFP16-split tiles: operands scaled by a per-tensor power of two and split into
  *    fp16 hi + lo (22 significant bits), the same three products at the fp16 rate; bound by the HBM
  *    stream of the activation operand.  `a_amax` / `g_amax` (optional device scalars, max |A| /
- *    max |G|, e.g. from the amax_out of the kernel that produced the operand) save the engine its
- *    own reduction pass over that operand; NULL = computed internally.  Accuracy is norm-relative
+ *    max |G| over the FINITE entries, e.g. from the amax_out of the kernel that produced the
+ *    operand) save the engine its own reduction pass over that operand; NULL = computed internally.
+ *    Every amax_out of this library and the internal reduction skip inf and NaN, so an operand with
+ *    a non-finite entry keeps its scale: inf stays inf, NaN stays NaN, and the other rows of the
+ *    result stay finite.  A supplied maximum smaller than the true one overflows the fp16 split;
+ *    a larger one costs precision.  Accuracy is norm-relative
  *    (elements > 2^23 below the tensor maximum lose relative precision).  engine 0 picks 3 for
  *    real contractions (n >= 32, k >= 16), 1 for thin ones.  On large operands (m >= 32 768) engine 3
  *    runs as clusters of two CTAs (tcgen05 cta_group::2, UMMA M = 256: each CTA stages its own 128

@@ -70,7 +70,7 @@ __global__ void __launch_bounds__(kColThreads) k_col_reduce(const ColArgs a, int
                         s2[q] += (double)yv[q] * (double)yv[q];
                     } else if (OP == COL_SUM) {
                         s1[q] += (double)yv[q];
-                        amx = fmaxf(amx, fabsf(yv[q]));
+                        amx = fmaxf(amx, finite_abs(yv[q]));
                     } else {
                         const float ctr = yv[q] - mu[q];
                         const float pre = fmaf(ctr, sc[q], sh[q]);
@@ -297,11 +297,11 @@ __global__ void __launch_bounds__(kEwThreads) k_bn_act_apply(const float* __rest
                 o.x = bn_lrelu(v.x, mu[0], sc[0], sh[0], slope); o.y = bn_lrelu(v.y, mu[1], sc[1], sh[1], slope);
                 o.z = bn_lrelu(v.z, mu[2], sc[2], sh[2], slope); o.w = bn_lrelu(v.w, mu[3], sc[3], sh[3], slope);
                 st4(z + r * ldz + ch, o);
-                amx = fmaxf(amx, fmaxf(fmaxf(fabsf(o.x), fabsf(o.y)), fmaxf(fabsf(o.z), fabsf(o.w))));
+                amx = fmaxf(amx, fmaxf(fmaxf(finite_abs(o.x), finite_abs(o.y)), fmaxf(finite_abs(o.z), finite_abs(o.w))));
             } else {
                 const float o = bn_lrelu(__ldg(y + r * ldy + ch), mu[0], sc[0], sh[0], slope);
                 z[r * ldz + ch] = o;
-                amx = fmaxf(amx, fabsf(o));
+                amx = fmaxf(amx, finite_abs(o));
             }
         }
     }
@@ -355,7 +355,7 @@ __global__ void __launch_bounds__(kEwThreads) k_bn_act_bwd_apply(const BwdArgs a
                 } else {
                     out[q] = sc[q] * da;
                 }
-                amx = fmaxf(amx, fabsf(out[q]));
+                amx = fmaxf(amx, finite_abs(out[q]));
             }
             if (VEC == 4) st4(a.dy + r * a.lddy + ch, make_float4(out[0], out[1], out[2], out[3]));
             else a.dy[r * a.lddy + ch] = out[0];

@@ -82,9 +82,18 @@ __device__ __forceinline__ Moments from_shifted(float n, float p, float s1, floa
 __device__ __forceinline__ float4 ldg4(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
 __device__ __forceinline__ void st4(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
 
+// |x| as it enters a published max |x|: inf and NaN count as 0.  The fp16-split engine scales an operand by a power of two
+// taken from that maximum; an inf there would leave the scale at 1 and overflow every finite entry above 65504 in the fp16
+// split, so rows without any inf would turn inf / NaN.  With the finite maximum an inf entry stays inf and a NaN stays NaN.
+__device__ __forceinline__ float finite_abs(float x) {
+    const float a = fabsf(x);
+    return a <= 3.402823466e+38f ? a : 0.f;
+}
+
 // max |x| of a produced tensor, published for the fp16-split GEMM engine that consumes it (sgb_gemm a_amax):
 // per-thread running maximum -> warp -> CTA -> one atomicMax on the float bits (non-negative floats order like
 // unsigned ints; max is order-independent, so the result is deterministic).  `scratch`: >= 32 uint32 of shared memory.
+// Callers accumulate `mx` with finite_abs.
 __device__ __forceinline__ void publish_amax(float mx, uint32_t* scratch, float* slot) {
     uint32_t b = __reduce_max_sync(0xffffffffu, __float_as_uint(mx));
     const int warp = threadIdx.x >> 5, nw = (blockDim.x + 31) >> 5;

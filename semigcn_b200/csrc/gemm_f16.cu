@@ -47,7 +47,8 @@ namespace sgb {
 // ------------------------------------------------------------------------------------------
 // per-tensor power-of-two scale from max |x|
 // ------------------------------------------------------------------------------------------
-// s = 2^(14 - floor(log2 amax)) -> amax * s in [2^14, 2^15); amax == 0 / non-finite -> 1
+// s = 2^(14 - floor(log2 amax)) -> amax * s in [2^14, 2^15); amax == 0 / non-finite -> 1 (every max |x| handed to the
+// engine is taken over the finite entries, so an inf or NaN operand entry does not reach here)
 __host__ __device__ __forceinline__ void f16_scale_from_amax(float amax, float& s, float& inv) {
     uint32_t bits;
 #ifdef __CUDA_ARCH__
@@ -69,8 +70,8 @@ __host__ __device__ __forceinline__ void f16_scale_from_amax(float amax, float& 
 #endif
 }
 
-// max |x| over an [m, c] matrix -> atomicMax on the float bits (non-negative floats order like uints).
-// The slot must be zero before the launch.
+// max |x| over the finite entries of an [m, c] matrix (finite_abs) -> atomicMax on the float bits (non-negative floats order
+// like uints).  The slot must be zero before the launch.
 __global__ void __launch_bounds__(256) k_amax(const float* __restrict__ x, int64_t ldx, int64_t m, int c, uint32_t* __restrict__ slot) {
     const int cv = c >> 2;
     const int64_t total = m * cv;
@@ -79,7 +80,7 @@ __global__ void __launch_bounds__(256) k_amax(const float* __restrict__ x, int64
         const int64_t r = i / cv;
         const int ch = (int)(i % cv) * 4;
         const float4 v = ldg4(x + r * ldx + ch);
-        mx = fmaxf(mx, fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w))));
+        mx = fmaxf(mx, fmaxf(fmaxf(finite_abs(v.x), finite_abs(v.y)), fmaxf(finite_abs(v.z), finite_abs(v.w))));
     }
     uint32_t b = __float_as_uint(mx);
     b = __reduce_max_sync(0xffffffffu, b);
@@ -155,7 +156,7 @@ struct HArgs {
 };
 
 // weights -> scale, hi/lo fp16 split, zero padded, in the exact per-stage shared-memory image.
-// Small grid; every CTA first reduces max |W| itself (W is at most 1 MB and L2-resident), so one launch
+// Small grid; every CTA first reduces max |W| (finite entries) itself (W is at most 1 MB and L2-resident), so one launch
 // does amax + prep and the scale never round-trips through the host.
 __global__ void __launch_bounds__(256) k_prep_weights_f16(const float* __restrict__ w, int64_t ldw, int transb, int n, int k, int bn,
                                                           int n_tiles, int k_chunks, __half* __restrict__ wp, float* __restrict__ wscale) {
@@ -165,11 +166,11 @@ __global__ void __launch_bounds__(256) k_prep_weights_f16(const float* __restric
     if (ldw == cols && (reinterpret_cast<uintptr_t>(w) & 15) == 0 && ((rows * cols) & 3) == 0) {       // dense, aligned: flat 128-bit scan
         for (int i = threadIdx.x; i < (rows * cols) >> 2; i += blockDim.x) {
             const float4 v = ldg4(w + 4 * i);
-            mx = fmaxf(mx, fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w))));
+            mx = fmaxf(mx, fmaxf(fmaxf(finite_abs(v.x), finite_abs(v.y)), fmaxf(finite_abs(v.z), finite_abs(v.w))));
         }
     } else {
         for (int r = 0; r < rows; ++r)
-            for (int i = threadIdx.x; i < cols; i += blockDim.x) mx = fmaxf(mx, fabsf(w[(int64_t)r * ldw + i]));
+            for (int i = threadIdx.x; i < cols; i += blockDim.x) mx = fmaxf(mx, finite_abs(w[(int64_t)r * ldw + i]));
     }
     mx = __uint_as_float(__reduce_max_sync(0xffffffffu, __float_as_uint(mx)));
     if ((threadIdx.x & 31) == 0) sm[threadIdx.x >> 5] = mx;

@@ -319,7 +319,7 @@ __global__ void __launch_bounds__(kSpmmThreads, (VEC * ITERS >= 8) ? (STATS ? SG
                         out.store(a.y + v * a.ldy + ch[t]);
                         if (a.amax) {
 #pragma unroll
-                            for (int q = 0; q < VEC; ++q) amx = fmaxf(amx, fabsf(out.v[q]));
+                            for (int q = 0; q < VEC; ++q) amx = fmaxf(amx, finite_abs(out.v[q]));
                         }
                         if (STATS) {
 #pragma unroll

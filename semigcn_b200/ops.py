@@ -43,10 +43,10 @@ AMAX_ATTR = "_sgb_amax"     # python attribute on an activation tensor: (device 
 
 
 def tag_amax(t: Tensor, amax_slot: Tensor) -> None:
-    """Attach the producer's max|t| to the tensor object, together with the tensor's version counter: any in-place edit
-    between two blocks (``x *= k``, ``x.add_(skip)``, an in-place activation in user code) bumps ``_version`` and makes the
-    tag stale -- ``amax_of`` then returns None and the GEMM engine reduces max|x| itself (a stale, too small maximum
-    would overflow the fp16 split silently)."""
+    """Attach the producer's max|t| (over the finite entries of t: inf and NaN are skipped) to the tensor object, together
+    with the tensor's version counter: any in-place edit between two blocks (``x *= k``, ``x.add_(skip)``, an in-place
+    activation in user code) bumps ``_version`` and makes the tag stale -- ``amax_of`` then returns None and the GEMM
+    engine reduces max|x| itself (a stale, too small maximum would overflow the fp16 split silently)."""
     setattr(t, AMAX_ATTR, (amax_slot, t._version))
 
 

@@ -151,11 +151,19 @@ def _sgcn_pair(conv, seed=314, skip=False):
     return ours.to(DEV), ref
 
 
-@pytest.mark.parametrize("conv", ["gcnconv", "chebconv"])
-@pytest.mark.parametrize("skip", [False, True])
-def test_sgcn_forward_backward_vs_oracle(conv, skip):
-    """Whole 13-block SGCN (util/networks.py) on a 1 002-vertex icosphere, three weight seeds.
-    Positions and loss must match the fp32 CPU oracle to 1e-5.
+# (icosphere frequency, weight seeds, skip, conv): 1 002 vertices run every transform on the CUDA-core tiles, 33 642 vertices
+# run them on the tcgen05 fp16-split CTA pairs (m >= 32 768)
+SGCN_CASES = ([pytest.param(10, (314, 1, 2), skip, conv, id=f"{skip}-{conv}") for skip in (False, True)
+               for conv in ("gcnconv", "chebconv")]
+              + [pytest.param(58, (314,), False, conv, id=f"n33642-False-{conv}") for conv in ("gcnconv", "chebconv")])
+
+
+@pytest.mark.parametrize("freq,seeds,skip,conv", SGCN_CASES)
+def test_sgcn_forward_backward_vs_oracle(freq, seeds, skip, conv):
+    """Whole 13-block SGCN (util/networks.py) on a 1 002-vertex icosphere with three weight seeds, and on a 33 642-vertex
+    one (the tensor-core path) with one.
+    Positions and loss must match the fp32 CPU oracle to 1e-5 (at 33 642 vertices, where the fp32 oracle is itself further
+    than that from fp64: be within max(1e-5, 2x the fp32 oracle's distance) of fp64).
     Gradients that crossed 13 BatchNorm + LeakyReLU layers are compared with an fp64 evaluation of the
     oracle.  In ANY fp32 implementation they carry amplified rounding noise plus discrete LeakyReLU
     "kink flips" (a pre-activation within rounding of zero takes the other branch than in fp64): the
@@ -165,11 +173,11 @@ def test_sgcn_forward_backward_vs_oracle(conv, skip):
     (seed, parameter) pairs ours is typically as close to fp64 as the fp32 oracle is.  The layer-level
     1e-5 bar is enforced per layer in the tests above."""
     from semigcn_b200.data import Data
-    prob = meshgen.synth_inpainting_problem(10, smooth_iters=10, n_dummy=4)
+    prob = meshgen.synth_inpainting_problem(freq, smooth_iters=10, n_dummy=4)
     mesh = prob["mesh"]
     dm = prob["vmask_dummy"][:, :1] * prob["v_mask"].float().reshape(-1, 1)
     rows = []
-    for seed in (314, 1, 2):
+    for seed in seeds:
         ours, ref = _sgcn_pair(conv, seed=seed, skip=skip)
         ref64 = copy.deepcopy(ref).double()
 
@@ -189,8 +197,18 @@ def test_sgcn_forward_backward_vs_oracle(conv, skip):
         loss = O.mask_pos_rec_loss(out, prob["ini_vs"].to(DEV), prob["v_mask"].to(DEV)) + \
             4.0 * O.mask_norm_rec_loss(O.compute_fn(out, mesh.faces.to(DEV)), prob["fn"].to(DEV), prob["f_mask"].to(DEV))
         loss.backward()
-        assert_close(out, out_r, REL_TOL, "positions")
-        assert abs(loss.item() - loss_r.item()) <= 1e-5 * abs(loss_r.item())
+        e_pos, e_pos32, e_pos64 = rel_err(out, out_r), rel_err(out_r, out_64), rel_err(out, out_64)
+        msg = f"positions: {e_pos:.2e} from the fp32 oracle, {e_pos64:.2e} from fp64 (the fp32 oracle: {e_pos32:.2e})"
+        if freq <= 10:
+            assert e_pos <= REL_TOL, msg
+            assert abs(loss.item() - loss_r.item()) <= 1e-5 * abs(loss_r.item())
+        else:
+            # 13 blocks at 33 642 vertices: the fp32 oracle itself is 1.6e-5 .. 3.0e-5 from fp64 (measured on a B200 host,
+            # ours 1.9e-5 .. 3.1e-5 from the fp32 oracle), so the truth is fp64 and the bar that of test_bn_near_constant_channels
+            assert e_pos64 <= max(REL_TOL, 2.0 * e_pos32), msg
+            e_loss32 = abs(loss_r.item() - loss_64.item())
+            assert abs(loss.item() - loss_64.item()) <= max(1e-5 * abs(loss_64.item()), 2.0 * e_loss32), \
+                f"loss {loss.item()!r}, fp32 oracle {loss_r.item()!r}, fp64 {loss_64.item()!r}"
 
         def check(name, g_ours, g_ref32, g_ref64):
             e_ours, e_ref = rel_err(g_ours, g_ref64), rel_err(g_ref32, g_ref64)
