@@ -293,6 +293,25 @@ SGB_API int sgb_bnf_loss_bwd(const float* fn, const float* new_fn, int64_t nf, i
  * ------------------------------------------------------------------------------------ */
 SGB_API int sgb_input_prep(const float* z1, int64_t ldz, int64_t n, const float* dm, float* x, float* scratch /* [16] */, void* stream);
 
+/* ------------------------------------------------------------------------------------ *
+ * 8. Point-to-surface distance: the accuracy metric of the inpainting evaluation (sgcn.py:183,193,
+ *    check/dist_check.py), exact nearest-triangle search over a uniform grid (surface_dist.cu).
+ *    dist[i] = min over all faces f of the Euclidean distance from points[i] to the closed triangle f,
+ *    face[i] = the face attaining it, the smallest face id among exact ties.  Zero-area faces (collinear
+ *    or coincident corners) are the union of their edge segments; duplicate faces and non-manifold soup
+ *    are valid; the target need not be closed.  Evaluated in fp64 on the fp32 coordinates; a query equal
+ *    to a target vertex gives exactly 0.  A query with a non-finite coordinate gives dist = NaN, face = -1.
+ *    tris [nf][12]: the corners of face f as floats 0..8 of row f (floats 9..11 unused), 16-byte aligned,
+ *    all finite.  The grid: cell (x, y, z) = [o + (x, y, z) h, o + (x+1, y+1, z+1) h], numbered
+ *    (z gy + y) gx + x; cell c lists faces cell_faces[cell_start[c] .. cell_start[c+1]) and must list every
+ *    face whose bounding box overlaps the cell (semigcn_b200/distance.py::SurfaceIndex builds it).
+ *    The result does not depend on the grid.  No floating-point atomics, no synchronisation.
+ * ------------------------------------------------------------------------------------ */
+SGB_API int sgb_point_surface_distance(const float* points, int64_t ldp, int64_t n, const float* tris /* [nf][12] */, int64_t nf,
+                                       const int32_t* cell_start /* [gx gy gz + 1] */, const int32_t* cell_faces,
+                                       float ox, float oy, float oz, float h, int gx, int gy, int gz,
+                                       float* dist /* [n] */, int32_t* face /* [n] */, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

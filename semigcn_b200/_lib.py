@@ -68,6 +68,8 @@ SIGNATURES = {
     "sgb_bnf_loss_fwd": (_i32, [_vp, _i64, _i64, _vp, _vp, _i64, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
     "sgb_bnf_loss_bwd": (_i32, [_vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp]),
     "sgb_lap_loss_bwd": (_i32, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]),
+    "sgb_point_surface_distance": (_i32, [_vp, _i64, _i64, _vp, _i64, _vp, _vp, _f32, _f32, _f32, _f32, _i32, _i32, _i32,
+                                          _vp, _vp, _vp]),
 }
 
 _lib: Optional[C.CDLL] = None
