@@ -142,9 +142,8 @@ SGB_API int sgb_gather_rows(const float* x, int64_t ldx, const int32_t* idx, int
 /* ------------------------------------------------------------------------------------ *
  * 3. Dense feature transform (the per-layer `lin` of GCNConv / `lins[k]` of ChebConv,
  *    nn.Linear of util/networks.py:35,52,58-61) and its two gradients.
- *    sgb_gemm:       C[m,n] (+)= f(A)[m,k] * op(B) + bias,  op(B) = B^T for transb=1
+ *    sgb_gemm:       C[m,n] (+)= A[m,k] * op(B) + bias,  op(B) = B^T for transb=1
  *                    (B is [n,k], i.e. a torch Linear weight) or B for transb=0 (B is [k,n]).
- *                    f = optional per-k-channel centred BatchNorm + LeakyReLU on A (as in sgb_spmm).
  *                    stat_partials: [sgb_gemm_stat_rows(m)][3][n] column (count, mean, M2) of C.
  *    sgb_gemm_tn:    D[n,k] (+)= G[m,n]^T * A[m,k]   (weight gradient; split over m with a
  *                    fixed-order two-stage reduction -> deterministic).
@@ -152,12 +151,12 @@ SGB_API int sgb_gather_rows(const float* x, int64_t ldx, const int32_t* idx, int
  *    stat_partials rows: every engine writes per-CTA (not per-tile) moments, at most
  *    sgb_gemm_stat_rows(m) = 4 * min(ceil(m/128), #SMs) rows, and zero-fills the rows it does not use
  *    (count 0 rows drop out of the merge) -- the finalisation cost no longer grows with m.
- *    `engine`: 0 = auto, 1 = fp32 CUDA-core tiles, 2 = tcgen05 3xTF32 tensor-core tiles
- *    (error-compensated: hi*hi + lo*hi + hi*lo, fp32 accumulate in TMEM).  The tensor-core
- *    engine stages the split / pre-tiled weights in `workspace` (sgb_gemm_workspace_bytes).
- *    3 = tcgen05 2xFP16-split tiles: operands scaled by a per-tensor power of two and split into
- *    fp16 hi + lo (22 significant bits), the same three products at the fp16 rate; bound by the HBM
- *    stream of the activation operand.  `a_amax` / `g_amax` (optional device scalars, max |A| /
+ *    `engine`: 0 = auto, 1 = fp32 CUDA-core tiles, 3 = tcgen05 2xFP16-split tiles (sgb_gemm_tn also
+ *    4, see below; any other value is SGB_EINVAL).  Engine 3 scales the operands by a per-tensor
+ *    power of two and splits them into fp16 hi + lo (22 significant bits); the error-compensated
+ *    products hi*hi + lo*hi + hi*lo accumulate in fp32 in TMEM.  It is bound by the HBM stream of the
+ *    activation operand, and sgb_gemm stages the split / pre-tiled weights in `workspace`
+ *    (sgb_gemm_workspace_bytes).  `a_amax` / `g_amax` (optional device scalars, max |A| /
  *    max |G| over the FINITE entries, e.g. from the amax_out of the kernel that produced the
  *    operand) save the engine its own reduction pass over that operand; NULL = computed internally.
  *    Every amax_out of this library and the internal reduction skip inf and NaN, so an operand with
@@ -177,7 +176,6 @@ SGB_API int sgb_gemm_stat_rows(int64_t m);
 SGB_API size_t sgb_gemm_workspace_bytes(int64_t m, int n, int k, int engine);
 SGB_API int sgb_gemm(int transb, const float* a, int64_t lda, const float* b, int64_t ldb,
              float* c, int64_t ldc, int64_t m, int n, int k,
-             const float* a_mean, const float* a_scale, const float* a_shift, float slope,
              const float* bias, int accumulate, float* stat_partials, const float* a_amax,
              void* workspace, size_t workspace_bytes, int engine, void* stream);
 SGB_API size_t sgb_gemm_tn_workspace_bytes(int64_t m, int n, int k);

@@ -17,7 +17,6 @@ CSRC = os.path.join(_HERE, "csrc")
 LIB_PATH = os.environ.get("SGB_LIB_PATH") or os.path.join(CSRC, "libsemigcn_b200.so")   # override: A/B builds of the same ABI
 
 MODE_GCN, MODE_CHEB, MODE_ADJ = 0, 1, 2
-ENGINE_AUTO, ENGINE_SIMT, ENGINE_TC = 0, 1, 2
 
 _i64, _i32, _f32, _vp, _sz = C.c_int64, C.c_int, C.c_float, C.c_void_p, C.c_size_t
 _f64 = C.c_double
@@ -40,8 +39,7 @@ SIGNATURES = {
     "sgb_gather_rows": (_i32, [_vp, _i64, _vp, _i64, _i32, _vp, _i64, _vp]),
     "sgb_gemm_stat_rows": (_i32, [_i64]),
     "sgb_gemm_workspace_bytes": (_sz, [_i64, _i32, _i32, _i32]),
-    "sgb_gemm": (_i32, [_i32, _vp, _i64, _vp, _i64, _vp, _i64, _i64, _i32, _i32, _vp, _vp, _vp, _f32, _vp, _i32,
-                        _vp, _vp, _vp, _sz, _i32, _vp]),
+    "sgb_gemm": (_i32, [_i32, _vp, _i64, _vp, _i64, _vp, _i64, _i64, _i32, _i32, _vp, _i32, _vp, _vp, _vp, _sz, _i32, _vp]),
     "sgb_gemm_tn_workspace_bytes": (_sz, [_i64, _i32, _i32]),
     "sgb_gemm_tn": (_i32, [_vp, _i64, _vp, _i64, _vp, _i64, _i64, _i32, _i32, _i32, _vp, _vp, _vp, _sz, _i32, _vp]),
     "sgb_colsum_workspace_bytes": (_sz, [_i64, _i32]),

@@ -109,14 +109,13 @@ __device__ __forceinline__ void publish_amax(float mx, uint32_t* scratch, float*
 // zero-fills the rest): 4 * min(ceil(m / 128), #SMs) -- gemm.cu
 int gemm_stat_rows(int64_t m);
 
-// arguments of the dense transform C (+)= f(A) op(B) + bias (see sgb_gemm)
+// arguments of the dense transform C (+)= A op(B) + bias (see sgb_gemm)
 struct GemmArgs {
     int transb;
     const float* a; int64_t lda;
     const float* b; int64_t ldb;
     float* c; int64_t ldc;
     int64_t m; int n; int k;
-    const float* a_mean; const float* a_scale; const float* a_shift; float slope;
     const float* bias; int accumulate; float* stat_partials;
 };
 

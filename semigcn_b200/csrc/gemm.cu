@@ -1,5 +1,5 @@
 // C-ABI entry points of the dense feature transform; dispatch between the fp32 CUDA-core
-// tiles (gemm_simt.cu) and the tcgen05 3xTF32 tiles (gemm_tc.cu).
+// tiles (gemm_simt.cu) and the tcgen05 fp16-split tiles (gemm_f16.cu).
 #include "common.cuh"
 
 namespace sgb {
@@ -7,14 +7,8 @@ int gemm_simt_launch(const GemmArgs& g, cudaStream_t stream);
 int gemm_tn_simt_launch(const float* g, int64_t ldg, const float* a, int64_t lda, float* d, int64_t ldd, int64_t m, int n, int k,
                         int accumulate, void* ws, size_t ws_bytes, cudaStream_t stream);
 size_t gemm_tn_simt_workspace(int64_t m, int n, int k);
-bool gemm_tc_supported(int64_t m, int n, int k, int64_t lda, int64_t ldc, const void* a, const void* c, const void* bias,
-                       const void* a_scale);
-size_t gemm_tc_workspace(int n, int k);
-int gemm_tc_launch(const GemmArgs& g, void* ws, size_t ws_bytes, cudaStream_t stream);
-bool gemm_tn_tc_supported(int64_t m, int n, int k, int64_t ldg, int64_t lda, const void* g, const void* a);
-size_t gemm_tn_tc_workspace(int64_t m, int n, int k);
-int gemm_tn_tc_launch(const float* g, int64_t ldg, const float* a, int64_t lda, float* d, int64_t ldd, int64_t m, int n, int k,
-                      int accumulate, void* ws, size_t ws_bytes, cudaStream_t stream);
+bool gemm_f16_supported(int64_t m, int n, int k, int64_t lda, int64_t ldc, const void* a, const void* c, const void* bias);
+bool gemm_tn_f16_supported(int64_t m, int n, int k, int64_t ldg, int64_t lda, const void* g, const void* a);
 size_t gemm_f16_workspace(int n, int k);
 int gemm_f16_launch(const GemmArgs& g, const float* a_amax, void* ws, size_t ws_bytes, cudaStream_t stream);
 size_t gemm_tn_f16_workspace(int64_t m, int n, int k);
@@ -47,54 +41,38 @@ int gemm_stat_rows(int64_t m) {
 extern "C" int sgb_gemm_stat_rows(int64_t m) { return gemm_stat_rows(m); }
 
 extern "C" size_t sgb_gemm_workspace_bytes(int64_t m, int n, int k, int engine) {
-    if (m < 0 || n <= 0 || k <= 0 || engine == 1) return 0;
-    if (engine == 0 && !tc_worthwhile(m, n, k)) return 0;
-    if (n % 16 != 0 || k % 4 != 0) return 0;
-    size_t w2 = gemm_tc_workspace(n, k), w3 = gemm_f16_workspace(n, k);
-    return engine == 2 ? w2 : engine == 3 ? w3 : (w2 > w3 ? w2 : w3);
+    if (m < 0 || n <= 0 || k <= 0 || n % 16 != 0 || k % 4 != 0) return 0;
+    if (engine == 3 || (engine == 0 && tc_worthwhile(m, n, k))) return gemm_f16_workspace(n, k);
+    return 0;
 }
 
 extern "C" int sgb_gemm(int transb, const float* a, int64_t lda, const float* b, int64_t ldb, float* c, int64_t ldc, int64_t m,
-                        int n, int k, const float* a_mean, const float* a_scale, const float* a_shift, float slope, const float* bias,
-                        int accumulate, float* stat_partials, const float* a_amax, void* workspace, size_t workspace_bytes, int engine,
-                        void* stream) {
+                        int n, int k, const float* bias, int accumulate, float* stat_partials, const float* a_amax, void* workspace,
+                        size_t workspace_bytes, int engine, void* stream) {
     SGB_CHECK_ARG(a && b && c && m >= 0 && n > 0 && k > 0, "sgb_gemm: bad argument m=%lld n=%d k=%d", (long long)m, n, k);
     SGB_CHECK_ARG(lda >= k && ldc >= n && ldb >= (transb ? k : n), "sgb_gemm: leading dimension too small");
-    SGB_CHECK_ARG((a_scale == nullptr) == (a_shift == nullptr) && (a_scale == nullptr) == (a_mean == nullptr),
-                  "sgb_gemm: a_mean / a_scale / a_shift must come together");
-    SGB_CHECK_ARG(engine >= 0 && engine <= 3, "sgb_gemm: bad engine %d", engine);
+    SGB_CHECK_ARG(engine == 0 || engine == 1 || engine == 3, "sgb_gemm: bad engine %d", engine);
     if (m == 0) return SGB_OK;
-    GemmArgs g{transb, a, lda, b, ldb, c, ldc, m, n, k, a_mean, a_scale, a_shift, slope, bias, accumulate, stat_partials};
-    const bool tc_ok = gemm_tc_supported(m, n, k, lda, ldc, a, c, bias, a_scale);
-    if (engine == 2) {
-        if (!tc_ok) {
-            set_error("sgb_gemm: tcgen05 engine needs n %% 16 == 0, k %% 4 == 0 and 16-byte aligned operands (n=%d k=%d)", n, k);
-            return SGB_ENOTSUP;
-        }
-        return gemm_tc_launch(g, workspace, workspace_bytes, (cudaStream_t)stream);
-    }
+    GemmArgs g{transb, a, lda, b, ldb, c, ldc, m, n, k, bias, accumulate, stat_partials};
+    const bool tc_ok = gemm_f16_supported(m, n, k, lda, ldc, a, c, bias);
     if (engine == 3) {
-        if (!tc_ok || a_scale) {
-            set_error("sgb_gemm: fp16-split engine needs n %% 16 == 0, k %% 4 == 0, 16-byte aligned operands and no A prologue (n=%d k=%d)", n, k);
+        if (!tc_ok) {
+            set_error("sgb_gemm: fp16-split engine needs n %% 16 == 0, k %% 4 == 0 and 16-byte aligned operands (n=%d k=%d)", n, k);
             return SGB_ENOTSUP;
         }
         return gemm_f16_launch(g, a_amax, workspace, workspace_bytes, (cudaStream_t)stream);
     }
-    if (engine == 0 && tc_ok && tc_worthwhile(m, n, k) && workspace) {
-        // auto: the fp16-split tiles (HBM-bound) unless the BatchNorm prologue is fused into the A load
-        if (!a_scale && workspace_bytes >= gemm_f16_workspace(n, k))
-            return gemm_f16_launch(g, a_amax, workspace, workspace_bytes, (cudaStream_t)stream);
-        if (workspace_bytes >= gemm_tc_workspace(n, k)) return gemm_tc_launch(g, workspace, workspace_bytes, (cudaStream_t)stream);
-    }
+    // auto: the fp16-split tiles (HBM-bound) for real contractions
+    if (engine == 0 && tc_ok && tc_worthwhile(m, n, k) && workspace && workspace_bytes >= gemm_f16_workspace(n, k))
+        return gemm_f16_launch(g, a_amax, workspace, workspace_bytes, (cudaStream_t)stream);
     return gemm_simt_launch(g, (cudaStream_t)stream);
 }
 
 extern "C" size_t sgb_gemm_tn_workspace_bytes(int64_t m, int n, int k) {
     if (m < 0 || n <= 0 || k <= 0) return 0;
-    size_t a = gemm_tn_simt_workspace(m, n, k), b = (n % 4 == 0 && k % 4 == 0) ? gemm_tn_tc_workspace(m, n, k) : 0;
+    size_t a = gemm_tn_simt_workspace(m, n, k);
     size_t c = (n % 4 == 0 && k % 4 == 0) ? gemm_tn_f16_workspace(m, n, k) : 0;
     size_t e = gemm_tn_pair_workspace(m, n, k);
-    a = a > b ? a : b;
     a = a > c ? a : c;
     return a > e ? a : e;
 }
@@ -104,8 +82,8 @@ extern "C" int sgb_gemm_tn(const float* g, int64_t ldg, const float* a, int64_t 
                            void* stream) {
     SGB_CHECK_ARG(g && a && d && m >= 0 && n > 0 && k > 0, "sgb_gemm_tn: bad argument");
     SGB_CHECK_ARG(ldg >= n && lda >= k && ldd >= k, "sgb_gemm_tn: leading dimension too small");
-    SGB_CHECK_ARG(engine >= 0 && engine <= 4, "sgb_gemm_tn: bad engine %d", engine);
-    const bool tc_ok = gemm_tn_tc_supported(m, n, k, ldg, lda, g, a);
+    SGB_CHECK_ARG(engine == 0 || engine == 1 || engine == 3 || engine == 4, "sgb_gemm_tn: bad engine %d", engine);
+    const bool tc_ok = gemm_tn_f16_supported(m, n, k, ldg, lda, g, a);
     // auto: 256-row multiples of D go to CTA pairs (measured on 998 562 vertices, amax supplied: n256_k256 0.517 -> 0.425 ms,
     // n512_k256 0.994 -> 0.839 ms, n256_k64 0.390 -> 0.310 ms against the single-CTA engine)
     if (engine == 0 && tc_ok && gemm_tn_pair_ok(m, n, k) && m >= 32768) engine = 4;
@@ -116,13 +94,6 @@ extern "C" int sgb_gemm_tn(const float* g, int64_t ldg, const float* a, int64_t 
         }
         return gemm_tn_pair_launch(g, ldg, a, lda, g_amax, a_amax, d, ldd, m, n, k, accumulate, workspace, workspace_bytes, (cudaStream_t)stream);
     }
-    if (engine == 2) {
-        if (!tc_ok) {
-            set_error("sgb_gemm_tn: tcgen05 engine needs n %% 4 == 0, k %% 4 == 0 and 16-byte aligned operands");
-            return SGB_ENOTSUP;
-        }
-        return gemm_tn_tc_launch(g, ldg, a, lda, d, ldd, m, n, k, accumulate, workspace, workspace_bytes, (cudaStream_t)stream);
-    }
     if (engine == 3 || (engine == 0 && tc_ok && tn_tc_worthwhile(m, n, k))) {
         if (!tc_ok) {
             set_error("sgb_gemm_tn: fp16-split engine needs n %% 4 == 0, k %% 4 == 0 and 16-byte aligned operands");
@@ -130,7 +101,5 @@ extern "C" int sgb_gemm_tn(const float* g, int64_t ldg, const float* a, int64_t 
         }
         return gemm_tn_f16_launch(g, ldg, a, lda, g_amax, a_amax, d, ldd, m, n, k, accumulate, workspace, workspace_bytes, (cudaStream_t)stream);
     }
-    if (engine == 0 && tc_ok && tn_tc_worthwhile(m, n, k))
-        return gemm_tn_tc_launch(g, ldg, a, lda, d, ldd, m, n, k, accumulate, workspace, workspace_bytes, (cudaStream_t)stream);
     return gemm_tn_simt_launch(g, ldg, a, lda, d, ldd, m, n, k, accumulate, workspace, workspace_bytes, (cudaStream_t)stream);
 }

@@ -3,10 +3,9 @@
 // Each fp32 operand is scaled by a per-tensor power of two s (exact) so that max |x s| lies in
 // [2^14, 2^15), then split   x s = hi + lo,  hi = rn_f16(x s),  lo = rn_f16(x s - hi)   (22 significant
 // bits), and the product is evaluated as   A*B ~= (A_lo*B_hi + A_hi*B_lo + A_hi*B_hi) / (s_A s_B)
-// with fp32 accumulation in TMEM.  Same three-product error compensation as the 3xTF32 engine
-// (gemm_tc.cu), but kind::f16 runs at twice the tf32 rate and every operand byte (shared memory,
-// L2 -> SM weight traffic) is halved: at these rates both kernels are bound by the HBM stream of the
-// activation operand, which is what the feature transform algorithmically has to read.
+// with fp32 accumulation in TMEM.  kind::f16 runs at twice the tf32 rate and every operand byte
+// (shared memory, L2 -> SM weight traffic) is half of a tf32 one: at these rates both kernels are bound
+// by the HBM stream of the activation operand, which is what the feature transform algorithmically has to read.
 // Accuracy contract: max |C - C_exact| <= ~4e-7 * sum_k |A||B| (norm-relative, like fp32 SIMT);
 // elements more than ~2^-23 below their tensor's maximum lose relative (not absolute) precision,
 // since fp16 has 5 exponent bits -- see DESIGN.md "engine 3".
@@ -25,22 +24,6 @@
 #include "umma.cuh"
 #include <cuda_fp16.h>
 #include <stdlib.h>
-
-// Ablation switches for tools/ablate_gemm.sh (timing experiments: which role bounds the pipeline?).  Each removes the WORK of one
-// role of k_gemm_f16 and keeps its barrier protocol, so the kernel still terminates; the results are garbage.  Never set in the
-// library build.
-#ifndef SGB_ABL
-#define SGB_ABL 0
-#endif
-#define SGB_ABL_NO_BCOPY 1      // weights copied for the first ring round only
-#define SGB_ABL_NO_STORE 2      // epilogue: no global stores
-#define SGB_ABL_NO_EPI 4        // epilogue: only the accumulator hand-shake
-#define SGB_ABL_NO_CONV 8       // converters: only the hand-shakes
-#define SGB_ABL_NO_TMA 16       // A loader: no TMA
-#define SGB_ABL_NO_MMA 32       // MMA issuer: no tcgen05.mma
-#define SGB_ABL_T_NO_MMA 64     // weight-gradient kernels: no tcgen05.mma
-#define SGB_ABL_T_NO_CONV 128   // weight-gradient kernels: converters only do the hand-shakes
-#define SGB_ABL_T_NO_DRAIN 256  // weight-gradient kernels: drain warps only do the hand-shakes
 
 namespace sgb {
 
@@ -248,7 +231,7 @@ __device__ __forceinline__ void h_epi_chunk(const HArgs& g, uint32_t taddr, floa
         const bool on = FULL || (col_ok && i * 4 + grp < nvalid);
         if (on) {
             o[i].x += b.x; o[i].y += b.y; o[i].z += b.z; o[i].w += b.w;
-            if (!(SGB_ABL & SGB_ABL_NO_STORE)) *reinterpret_cast<float4*>(cp + i * ld4) = o[i];
+            *reinterpret_cast<float4*>(cp + i * ld4) = o[i];
         }
     }
     if (stats) {
@@ -383,7 +366,7 @@ __global__ void __launch_bounds__(kHThreads, 1) k_gemm_f16(const __grid_constant
             const uint8_t* raw = raw_base + (size_t)rs * kHRawBytes;
             uint4 h[RPT], l[RPT];
 #pragma unroll
-            for (int hf = 0; hf < ((SGB_ABL & SGB_ABL_NO_CONV) ? 0 : 2); ++hf) {
+            for (int hf = 0; hf < 2; ++hf) {
                 float4 v[HALF][2];
 #pragma unroll
                 for (int i = 0; i < HALF; ++i) {
@@ -409,7 +392,7 @@ __global__ void __launch_bounds__(kHThreads, 1) k_gemm_f16(const __grid_constant
             uint8_t* a_hi = op_base + (size_t)s * stage_bytes;
             uint8_t* a_lo = a_hi + kHATile;
 #pragma unroll
-            for (int i = 0; i < ((SGB_ABL & SGB_ABL_NO_CONV) ? 0 : RPT); ++i) {
+            for (int i = 0; i < RPT; ++i) {
                 const int r = r0 + RSTEP * i;
                 const uint32_t off = (uint32_t)(r >> 3) * kHASbo + (uint32_t)cq * kHALbo + (uint32_t)(r & 7) * 16;
                 *reinterpret_cast<uint4*>(a_hi + off) = h[i];
@@ -440,11 +423,8 @@ __global__ void __launch_bounds__(kHThreads, 1) k_gemm_f16(const __grid_constant
                 const int m0 = (int)SGB_H_M0_OF(tile);
                 for (uint32_t q = 0; q < k_chunks; ++q) {
                     mbar_wait(&rempty[rs], rph ^ 1);
-                    if (SGB_ABL & SGB_ABL_NO_TMA) { mbar_arrive(&rfull[rs]); }
-                    else {
-                        mbar_arrive_expect_tx(&rfull[rs], kHRawBytes);
-                        tma_load_2d(raw_base + (size_t)rs * kHRawBytes, &g.a_map, (int)(q * kHBK), m0, &rfull[rs]);
-                    }
+                    mbar_arrive_expect_tx(&rfull[rs], kHRawBytes);
+                    tma_load_2d(raw_base + (size_t)rs * kHRawBytes, &g.a_map, (int)(q * kHBK), m0, &rfull[rs]);
                     if (++rs == raw_stages) { rs = 0; rph ^= 1; }
                 }
             }
@@ -466,8 +446,7 @@ __global__ void __launch_bounds__(kHThreads, 1) k_gemm_f16(const __grid_constant
                         mbar_arrive_expect_tx(&bfull[s], 2 * half_bytes);
                         bulk_g2s(b_dst, src_half + (size_t)q * 2 * b_tile_bytes, half_bytes, &bfull[s]);
                         bulk_g2s(b_dst + b_smem_bytes, src_half + (size_t)q * 2 * b_tile_bytes + b_tile_bytes, half_bytes, &bfull[s]);
-                    } else if ((SGB_ABL & SGB_ABL_NO_BCOPY) && (t * k_chunks + q) >= stages) { mbar_arrive(&full[s]); }
-                    else {
+                    } else {
                         mbar_arrive_expect_tx(&full[s], 2 * b_tile_bytes);
                         bulk_g2s(b_dst, src0 + (size_t)q * 2 * b_tile_bytes, 2 * b_tile_bytes, &full[s]);
                     }
@@ -496,7 +475,7 @@ __global__ void __launch_bounds__(kHThreads, 1) k_gemm_f16(const __grid_constant
                     const uint32_t b_hi = a_hi + 2 * kHATile;
                     const uint32_t b_lo = b_hi + b_smem_bytes;
 #pragma unroll
-                    for (int j = 0; j < ((SGB_ABL & SGB_ABL_NO_MMA) ? 0 : kHBK / 16); ++j) {
+                    for (int j = 0; j < kHBK / 16; ++j) {
                         const uint64_t dah = make_desc(a_hi + j * 2 * kHALbo, kHALbo, kHASbo);
                         const uint64_t dal = make_desc(a_lo + j * 2 * kHALbo, kHALbo, kHASbo);
                         const uint64_t dbh = make_desc(b_hi + j * 2 * kHBLbo, kHBLbo, kHBSbo);
@@ -559,7 +538,7 @@ __global__ void __launch_bounds__(kHThreads, 1) k_gemm_f16(const __grid_constant
 #pragma unroll
             for (int t = 0; t < 4; ++t) {            // unrolled: the moment registers are indexed statically
                 const int c0 = (2 * t + half) * 32;
-                if (c0 < ncols && !(SGB_ABL & SGB_ABL_NO_EPI)) {
+                if (c0 < ncols) {
                     float bm[4], bq[4];
                     const bool col_ok = c0 + cc < ncols;             // ncols is a multiple of 16 => whole float4 valid
                     const float* bias_p = g.bias ? g.bias + n0 + c0 + cc : nullptr;
@@ -607,7 +586,7 @@ __global__ void __launch_bounds__(kHThreads, 1) k_gemm_f16(const __grid_constant
 #undef SGB_H_M0_OF
 }
 
-// fixed-order split reduction -- gemm_tc.cu
+// fixed-order split reduction -- gemm_simt.cu
 int reduce_splits_launch(const float* partial, int splits, int n, int k, float* d, int64_t ldd, int accumulate, cudaStream_t stream);
 
 // ------------------------------------------------------------------------------------------
@@ -739,10 +718,7 @@ __global__ void __launch_bounds__(kTThreads, 1) k_gemm_tn_f16(const __grid_const
             mbar_wait(&rfull[rs], rph);
             const uint8_t* raw = raw_base + (size_t)rs * raw_bytes + raw_off;
             uint4 h[4], l[4];
-            if (SGB_ABL & SGB_ABL_T_NO_CONV) {
-#pragma unroll
-                for (int q = 0; q < 4; ++q) { h[q] = make_uint4(0u, 0u, 0u, 0u); l[q] = make_uint4(0u, 0u, 0u, 0u); }
-            } else if (col_ok) {
+            if (col_ok) {
                 float4 v[8];
 #pragma unroll
                 for (int r = 0; r < 8; ++r) v[r] = *reinterpret_cast<const float4*>(raw + (size_t)r * box * 4);
@@ -763,7 +739,7 @@ __global__ void __launch_bounds__(kTThreads, 1) k_gemm_tn_f16(const __grid_const
             fence_proxy_async();
             mbar_arrive(&rempty[rs]);
             mbar_wait(&empty[s], ph ^ 1);
-            if (in_tile && !(SGB_ABL & SGB_ABL_T_NO_CONV)) {
+            if (in_tile) {
                 uint8_t* st = op_base + (size_t)s * stage_bytes + base_off;
 #pragma unroll
                 for (int q = 0; q < 4; ++q) {
@@ -814,7 +790,7 @@ __global__ void __launch_bounds__(kTThreads, 1) k_gemm_tn_f16(const __grid_const
                 const uint32_t a_hi = g_lo + kTGTile;
                 const uint32_t a_lo = a_hi + a_tile_bytes;
 #pragma unroll
-                for (int j = 0; j < ((SGB_ABL & SGB_ABL_T_NO_MMA) ? 0 : kTBV / 16); ++j) {
+                for (int j = 0; j < kTBV / 16; ++j) {
                     const uint64_t dgh = make_desc(g_hi + j * 2 * kTLbo, kTLbo, kTSbo);
                     const uint64_t dgl = make_desc(g_lo + j * 2 * kTLbo, kTLbo, kTSbo);
                     const uint64_t dah = make_desc(a_hi + j * 2 * kTLbo, kTLbo, kTSbo);
@@ -847,7 +823,7 @@ __global__ void __launch_bounds__(kTThreads, 1) k_gemm_tn_f16(const __grid_const
             mbar_wait(&tfull[acc], (seg >> 1) & 1);
             tc_fence_after();
             const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(acc * t.acc_stride);
-            for (int c0 = 0; c0 < ((SGB_ABL & SGB_ABL_T_NO_DRAIN) ? 0 : kcols); c0 += 32) {
+            for (int c0 = 0; c0 < kcols; c0 += 32) {
                 float v[32];
                 tmem_ld_32x32(taddr + (uint32_t)c0, v);          // lane = row of D, registers = 32 consecutive columns
 #pragma unroll
@@ -1001,10 +977,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kPThreads, 1) k_gemm
             mbar_wait(&rfull[rs], rph);
             const uint8_t* raw = raw_base + (size_t)rs * raw_bytes + raw_off;
             uint4 h[4], l[4];
-            if (SGB_ABL & SGB_ABL_T_NO_CONV) {
-#pragma unroll
-                for (int q = 0; q < 4; ++q) { h[q] = make_uint4(0u, 0u, 0u, 0u); l[q] = make_uint4(0u, 0u, 0u, 0u); }
-            } else if (in_tile) {
+            if (in_tile) {
                 float4 v[8];
 #pragma unroll
                 for (int r = 0; r < 8; ++r) v[r] = *reinterpret_cast<const float4*>(raw + (size_t)r * box * 4);
@@ -1021,7 +994,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kPThreads, 1) k_gemm
             fence_proxy_async();                 // the conversion consumed the loaded values: the raw slot may go back to the TMA engine
             mbar_arrive(&rempty[rs]);
             mbar_wait(&empty[s], ph ^ 1);        // multicast commit of the leader's MMAs that read this slot (in BOTH CTAs)
-            if (in_tile && !(SGB_ABL & SGB_ABL_T_NO_CONV)) {
+            if (in_tile) {
                 uint8_t* st = op_base + (size_t)s * stage_bytes + base_off;
 #pragma unroll
                 for (int q = 0; q < 4; ++q) {
@@ -1070,7 +1043,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kPThreads, 1) k_gemm
                 const uint32_t a_hi = g_lo + kTGTile;
                 const uint32_t a_lo = a_hi + a_tile_bytes;
 #pragma unroll
-                for (int j = 0; j < ((SGB_ABL & SGB_ABL_T_NO_MMA) ? 0 : kTBV / 16); ++j) {
+                for (int j = 0; j < kTBV / 16; ++j) {
                     const uint64_t dgh = make_desc(g_hi + j * 2 * kTLbo, kTLbo, kTSbo);
                     const uint64_t dgl = make_desc(g_lo + j * 2 * kTLbo, kTLbo, kTSbo);
                     const uint64_t dah = make_desc(a_hi + j * 2 * kTLbo, kTLbo, kTSbo);
@@ -1104,7 +1077,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kPThreads, 1) k_gemm
             mbar_wait(&tfull[acc], (seg >> 1) & 1);
             tc_fence_after();
             const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(acc * t.acc_stride);
-            for (int c0 = 0; c0 < ((SGB_ABL & SGB_ABL_T_NO_DRAIN) ? 0 : kcols); c0 += 32) {
+            for (int c0 = 0; c0 < kcols; c0 += 32) {
                 float v[32];
                 tmem_ld_32x32(taddr + (uint32_t)c0, v);          // lane = row of D, registers = 32 consecutive columns
 #pragma unroll
@@ -1151,8 +1124,16 @@ struct HPlan {
     bool pair;
 };
 
+// what the forward kernels take: n a multiple of 16, 16-byte aligned rows of A and C (TMA loads, float4 stores)
+bool gemm_f16_supported(int64_t m, int n, int k, int64_t lda, int64_t ldc, const void* a, const void* c, const void* bias) {
+    auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
+    return n >= 16 && n % 16 == 0 && k >= 8 && k % 4 == 0 && lda % 4 == 0 && ldc % 4 == 0 && al16(a) && al16(c) &&
+           (!bias || al16(bias)) && m >= 1;
+}
+
 // CTA pairs: every n-tile must split into two halves of whole core-matrix rows (ncols % 16 == 0), and there must be enough
-// m-tiles to keep 74 pairs busy; SGB_F16_PAIR=0 / 1 overrides (experiments)
+// m-tiles to keep 74 pairs busy.  SGB_F16_PAIR=0 / 1 forces the single-CTA / pair kernel (from m > 128 rows), so that
+// tests and tools/bench_small_shapes.py can run both on small operands.
 static bool h_pair_wanted(int64_t m, int n) {
     if (m <= kHBM) return false;                 // a single m-tile: nothing to pair
     if (const char* e = getenv("SGB_F16_PAIR")) return atoi(e) != 0 && n % 16 == 0 && n >= 32;
@@ -1167,10 +1148,8 @@ static HPlan h_plan(int n, int k, bool pair = false) {
     p.k_chunks = (k + kHBK - 1) / kHBK;
     int sb = pair ? h_stage_bytes_pair(p.bn) : h_stage_bytes(p.bn);
     p.raw_stages = 3;
-    if (const char* e = getenv("SGB_F16_RAW")) { int v = atoi(e); if (v >= 2 && v <= kHMaxRawStages) p.raw_stages = v; }
     int st = (kHSmemBudget - kHBarBytes - kHEpiBytes - p.raw_stages * kHRawBytes - 1024) / sb;
     p.stages = st > kHMaxStages ? kHMaxStages : st;
-    if (const char* e = getenv("SGB_F16_STAGES")) { int v = atoi(e); if (v >= 2 && v <= p.stages) p.stages = v; }
     p.smem_bytes = (size_t)p.raw_stages * kHRawBytes + (size_t)p.stages * sb + kHBarBytes + kHEpiBytes;
     p.img_bytes = (size_t)p.n_tiles * p.k_chunks * 2 * h_b_tile_bytes(p.bn);
     p.acc_stride = (p.bn + 31) / 32 * 32;
@@ -1278,9 +1257,7 @@ static TPlan t_plan(int64_t m, int n, int k) {
     // boxes (32 vertices x (n + k) floats), so two stages left them latency-bound (~0.17 ms whatever the shape): as deep as fits, <= 8.
     int rs = (kHSmemBudget - kTBarBytes - kTEpiBytes - p.stages * sb) / raw;
     p.raw_stages = rs > kTMaxRawStages ? kTMaxRawStages : (rs < kTRawStages ? kTRawStages : rs);
-    if (const char* e = getenv("SGB_TN_RAW")) { int v = atoi(e); if (v >= 2 && v <= p.raw_stages) p.raw_stages = v; }
     p.conv_groups = (p.gbox + p.abox <= kTProducerWarps * 32 / 2 && p.stages >= 2 && p.raw_stages >= 2) ? 2 : 1;
-    if (const char* e = getenv("SGB_TN_GROUPS")) { if (atoi(e) == 1) p.conv_groups = 1; }
     p.smem_bytes = (size_t)p.raw_stages * raw + (size_t)p.stages * sb + kTBarBytes + kTEpiBytes;
     int tiles = p.k_tiles * p.n_tiles;
     int64_t want = num_sms() / tiles;
@@ -1297,6 +1274,12 @@ static TPlan t_plan(int64_t m, int n, int k) {
 }
 
 size_t gemm_tn_f16_workspace(int64_t m, int n, int k) { return t_plan(m, n, k).ws_bytes; }
+
+// what both weight-gradient kernels take: 16-byte aligned rows of G and A (TMA loads)
+bool gemm_tn_f16_supported(int64_t m, int n, int k, int64_t ldg, int64_t lda, const void* g, const void* a) {
+    auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
+    return n % 4 == 0 && k % 4 == 0 && ldg % 4 == 0 && lda % 4 == 0 && al16(g) && al16(a) && m >= 1;
+}
 
 int gemm_tn_f16_launch(const float* g, int64_t ldg, const float* a, int64_t lda, const float* g_amax, const float* a_amax, float* d,
                        int64_t ldd, int64_t m, int n, int k, int accumulate, void* ws, size_t ws_bytes, cudaStream_t stream) {
@@ -1361,7 +1344,6 @@ static PPlan p_plan(int64_t m, int n, int k) {
     const int sb = 2 * kTGTile + 2 * t_a_tile_bytes(p.ah);
     const int raw = (kTBV * (kTBM + p.ah) * 4 + 127) / 128 * 128;
     p.raw_stages = 3;
-    if (const char* e = getenv("SGB_PAIR_RAW")) { int v = atoi(e); if (v >= 2 && v <= kPMaxRawStages) p.raw_stages = v; }
     int st = (kHSmemBudget - 256 - kTEpiBytes - p.raw_stages * raw) / sb;
     p.stages = st > kHMaxStages ? kHMaxStages : st;
     p.smem_bytes = (size_t)p.raw_stages * raw + (size_t)p.stages * sb + 256 + kTEpiBytes;

@@ -2,9 +2,9 @@
 //
 // Replaces F.linear inside GCNConv.lin / ChebConv.lins[k] / nn.Linear (util/networks.py:25,35,
 // 42,52,58-61) at widths where the contraction is too thin for the tensor pipe (K or N < 64,
-// SURVEY.md §8(d)) and serves as the always-available exact-fp32 path; the tcgen05 3xTF32
-// tiles live in gemm_tc.cu.  Fused: BatchNorm-affine + LeakyReLU prologue on A, bias and
-// per-tile BatchNorm statistics in the epilogue (no extra pass over C).
+// SURVEY.md §8(d)) and serves as the always-available exact-fp32 path; the tcgen05 fp16-split
+// tiles live in gemm_f16.cu.  Fused: bias and per-tile BatchNorm statistics in the epilogue
+// (no extra pass over C).
 #include "common.cuh"
 
 namespace sgb {
@@ -24,7 +24,6 @@ __global__ void __launch_bounds__(kGemmThreads) k_gemm_simt(const GemmArgs g) {
     const int tid = threadIdx.x;
     const int tx = tid % 16, ty = tid / 16;
     const int n0 = blockIdx.y * BN;
-    const bool pro = g.a_scale != nullptr;
     const bool a_vec = (g.lda % 4 == 0) && ((reinterpret_cast<uintptr_t>(g.a) & 15) == 0);
     const bool b_vec = (g.ldb % 4 == 0) && ((reinterpret_cast<uintptr_t>(g.b) & 15) == 0);
 
@@ -59,12 +58,6 @@ __global__ void __launch_bounds__(kGemmThreads) k_gemm_simt(const GemmArgs g) {
 #pragma unroll
                     for (int q = 0; q < 4; ++q)
                         if (k0 + kq + q < g.k) v[q] = __ldg(p + q);
-                }
-                if (pro) {
-#pragma unroll
-                    for (int q = 0; q < 4; ++q)
-                        if (k0 + kq + q < g.k)
-                            v[q] = bn_lrelu(v[q], __ldg(g.a_mean + k0 + kq + q), __ldg(g.a_scale + k0 + kq + q), __ldg(g.a_shift + k0 + kq + q), g.slope);
                 }
             }
 #pragma unroll
@@ -298,6 +291,16 @@ __global__ void k_reduce_splits(const float* __restrict__ partial, int splits, i
     }
 }
 
+// D (+)= the sum of `splits` partial [n, k] tiles, added in split order (deterministic); also ends the tcgen05 weight
+// gradients of gemm_f16.cu
+int reduce_splits_launch(const float* partial, int splits, int n, int k, float* d, int64_t ldd, int accumulate, cudaStream_t stream) {
+    const int64_t total = (int64_t)n * k;
+    const int rgrid = (int)min64(ceil_div(total, 256), (int64_t)num_sms() * 8);
+    k_reduce_splits<<<rgrid, 256, 0, stream>>>(partial, splits, n, k, d, ldd, accumulate);
+    SGB_CHECK_LAUNCH("k_reduce_splits");
+    return SGB_OK;
+}
+
 // ---------------------------------------------------------------------------------------
 // Thin weight gradient  D[n,k] = sum_m G[m,n] A[m,k]  with n <= 32, k <= 64 (the 4-16-32 / 32-16-3 ends of the SGCN
 // stack): a pure HBM stream of two narrow matrices.  A CTA walks a contiguous row range in 32-row stages
@@ -448,11 +451,7 @@ int gemm_tn_simt_launch(const float* g, int64_t ldg, const float* a, int64_t lda
         SGB_THIN_CASE(4, 1) SGB_THIN_CASE(4, 2) SGB_THIN_CASE(16, 1) SGB_THIN_CASE(16, 2) SGB_THIN_CASE(32, 1) SGB_THIN_CASE(32, 2)
 #undef SGB_THIN_CASE
         SGB_CHECK_LAUNCH("k_gemm_tn_thin");
-        int64_t total = (int64_t)n * k;
-        int rgrid = (int)min64(ceil_div(total, 256), (int64_t)num_sms() * 8);
-        k_reduce_splits<<<rgrid, 256, 0, stream>>>((const float*)ws, grid, n, k, d, ldd, accumulate);
-        SGB_CHECK_LAUNCH("k_reduce_splits");
-        return SGB_OK;
+        return reduce_splits_launch((const float*)ws, grid, n, k, d, ldd, accumulate, stream);
     }
     int splits = tn_splits(m, n, k);
     size_t need = (size_t)splits * n * k * sizeof(float);
@@ -464,11 +463,7 @@ int gemm_tn_simt_launch(const float* g, int64_t ldg, const float* a, int64_t lda
     dim3 grid((unsigned)(ceil_div(n, kTnTile) * ceil_div(k, kTnTile)), (unsigned)splits);
     k_gemm_tn_partial<<<grid, 256, 0, stream>>>(g, ldg, a, lda, m, n, k, mps, (float*)ws);
     SGB_CHECK_LAUNCH("k_gemm_tn_partial");
-    int64_t total = (int64_t)n * k;
-    int rgrid = (int)min64(ceil_div(total, 256), (int64_t)num_sms() * 8);
-    k_reduce_splits<<<rgrid, 256, 0, stream>>>((const float*)ws, splits, n, k, d, ldd, accumulate);
-    SGB_CHECK_LAUNCH("k_reduce_splits");
-    return SGB_OK;
+    return reduce_splits_launch((const float*)ws, splits, n, k, d, ldd, accumulate, stream);
 }
 
 size_t gemm_tn_simt_workspace(int64_t m, int n, int k) {

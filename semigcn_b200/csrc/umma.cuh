@@ -1,4 +1,4 @@
-// tcgen05 / TMEM / mbarrier / bulk-copy PTX wrappers shared by the tensor-core GEMM engines (sm_100a only).
+// tcgen05 / TMEM / mbarrier / bulk-copy / TMA PTX wrappers of the fp16-split tensor-core GEMM (gemm_f16.cu; sm_100a only).
 #pragma once
 #include "common.cuh"
 #include <cuda.h>
@@ -50,16 +50,6 @@ __device__ __forceinline__ void tmem_dealloc(uint32_t addr, uint32_t cols) {
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(addr), "r"(cols) : "memory");
 }
 
-__device__ __forceinline__ void umma_tf32(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t"
-        "}" ::"r"(d_tmem),
-        "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
@@ -82,16 +72,6 @@ __device__ __forceinline__ void tmem_ld_32x32(uint32_t taddr, float* v) {
     for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
 }
 
-// hi = x rounded to nearest tf32 (10 explicit mantissa bits; ties away from zero), computed on the integer
-// pipe: adding half an ulp to the magnitude bits and masking is exactly cvt.rna.tf32.f32 for finite x, in 2
-// full-rate ops (ptxas expands the cvt into ~10 ops with NaN handling, which made the producers ALU-bound).
-// lo = x - hi is exact in fp32 and is fed to the tensor core as is: the hardware drops the bits below tf32
-// precision, an error <= 2^-10 |lo| <= 2^-21 |x|.
-__device__ __forceinline__ void split_tf32(float x, float& hi, float& lo) {
-    hi = __uint_as_float((__float_as_uint(x) + 0x1000u) & 0xFFFFE000u);
-    lo = x - hi;
-}
-
 // shared-memory matrix descriptor, no swizzle (cute::UMMA::SmemDescriptor: start>>4 [0,14), LBO>>4 [16,30),
 // SBO>>4 [32,46), version=1 [46,48), layout_type=0 [61,64))
 __device__ __forceinline__ uint64_t make_desc(uint32_t smem_addr, uint32_t lbo_bytes, uint32_t sbo_bytes, uint32_t layout_type = 0) {
@@ -103,15 +83,8 @@ __device__ __forceinline__ uint64_t make_desc(uint32_t smem_addr, uint32_t lbo_b
     return d;
 }
 
-// instruction descriptor (cute::UMMA::InstrDescriptor): c_format F32 = 1 @4, a/b_format TF32 = 2 @7/@10,
-// a_major @15, b_major @16 (0 = K-major, 1 = MN-major), n>>3 @17, m>>4 @24
-__host__ __device__ constexpr uint32_t make_idesc_tf32(int m, int n, int a_mn_major, int b_mn_major) {
-    return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)a_mn_major << 15) | ((uint32_t)b_mn_major << 16) |
-           ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
-}
-
-
-// kind::f16 (fp16 operands, fp32 accumulate): same descriptor layout, a/b_format F16 = 0
+// instruction descriptor (cute::UMMA::InstrDescriptor) of kind::f16 with fp16 operands and fp32 accumulate: c_format F32 = 1 @4,
+// a/b_format F16 = 0 @7/@10, a_major @15, b_major @16 (0 = K-major, 1 = MN-major), n>>3 @17, m>>4 @24
 __host__ __device__ constexpr uint32_t make_idesc_f16(int m, int n, int a_mn_major, int b_mn_major) {
     return (1u << 4) | ((uint32_t)a_mn_major << 15) | ((uint32_t)b_mn_major << 16) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
 }

@@ -238,10 +238,10 @@ def spmm(g: MeshGraph, x: Tensor, transpose: bool = False, in_affine: Affine = N
     return (y, partials) if want_stats else y
 
 
-def gemm(a: Tensor, b: Tensor, transb: bool = True, a_affine: Affine = None, bias: Optional[Tensor] = None,
+def gemm(a: Tensor, b: Tensor, transb: bool = True, bias: Optional[Tensor] = None,
          out: Optional[Tensor] = None, accumulate: bool = False, want_stats: bool = False, engine: int = 0,
          a_amax: Optional[Tensor] = None):
-    """C (+)= f(A) @ (B^T if transb else B) + bias.  ``a_amax``: optional device scalar max|A| (from the kernel
+    """C (+)= A @ (B^T if transb else B) + bias.  ``a_amax``: optional device scalar max|A| (from the kernel
     that produced A) for the fp16-split tensor-core engine; None = the engine reduces it itself."""
     lib = L.load()
     require_cuda(a, b, bias)
@@ -254,14 +254,13 @@ def gemm(a: Tensor, b: Tensor, transb: bool = True, a_affine: Affine = None, bia
     partials = None
     if want_stats:
         partials = torch.empty((lib.sgb_gemm_stat_rows(m), 3, n), dtype=torch.float32, device=a.device)
-    mu, sc, sh, slope = (a_affine if a_affine is not None else (None, None, None, 0.0))
     sp = _prof.span(f"gemm_n{n}_k{k}", 4.0 * (m * (k + n) + k * n + (m * n if accumulate else 0)), 2.0 * m * n * k) \
         if _prof.ACTIVE is not None else None
     wsb = lib.sgb_gemm_workspace_bytes(m, n, k, engine)
     ws = _ws(wsb, a.device) if wsb else None
     with torch.cuda.device(a.device):
         check(lib.sgb_gemm(1 if transb else 0, ptr(a), a.stride(0), ptr(b), b.stride(0), ptr(c), c.stride(0), m, n, k,
-                           ptr(mu), ptr(sc), ptr(sh), float(slope), ptr(bias), 1 if accumulate else 0, ptr(partials),
+                           ptr(bias), 1 if accumulate else 0, ptr(partials),
                            ptr(a_amax), ptr(ws), wsb, engine, stream_ptr(a.device)), "sgb_gemm")
     if sp is not None:
         sp.close()

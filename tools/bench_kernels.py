@@ -35,20 +35,16 @@ if 'spmm' in what.split(','):
 if 'gemm' in what.split(','):
     for (k, nn) in ((64, 128), (128, 256), (256, 256), (256, 512), (512, 256), (256, 128), (128, 64)):
         a = torch.randn(n, k, device=dev); w = torch.randn(nn, k, device=dev)
-        for eng in (2, 3):
-            ms = timeit(lambda: ops.gemm(a, w, engine=eng), reps=3, warm=1)
-            print(f'gemm k={k} n={nn} engine={eng}: {ms:7.3f} ms  {2.0 * n * k * nn / ms / 1e9:7.1f} TFLOP/s  {4.0 * n * (k + nn) / ms / 1e6:7.1f} GB/s')
+        ms = timeit(lambda: ops.gemm(a, w, engine=3), reps=3, warm=1)
+        print(f'gemm k={k} n={nn} engine=3: {ms:7.3f} ms  {2.0 * n * k * nn / ms / 1e9:7.1f} TFLOP/s  {4.0 * n * (k + nn) / ms / 1e6:7.1f} GB/s')
         amx = a.abs().max().reshape(1)
         ms3 = timeit(lambda: ops.gemm(a, w, engine=3, a_amax=amx), reps=3, warm=1)
         print(f'     engine 3 with a_amax supplied: {ms3:7.3f} ms  {4.0 * n * (k + nn) / ms3 / 1e6:7.1f} GB/s')
-        ms = timeit(lambda: ops.gemm(a, w, engine=2, want_stats=True), reps=3, warm=1)
-        print(f'     +stats: {ms:7.3f} ms')
 if 'gemm_tn' in what:
     for (k, nn) in ((64, 128), (128, 256), (256, 256), (256, 512), (512, 256), (256, 128), (128, 64)):
         a = torch.randn(n, k, device=dev); g_ = torch.randn(n, nn, device=dev)
-        for eng in (2, 3):
-            ms = timeit(lambda: ops.gemm_tn(g_, a, engine=eng), reps=3, warm=1)
-            print(f'gemm_tn k={k} n={nn} engine={eng}: {ms:7.3f} ms  {2.0 * n * k * nn / ms / 1e9:7.1f} TFLOP/s  {4.0 * n * (k + nn) / ms / 1e6:7.1f} GB/s')
+        ms = timeit(lambda: ops.gemm_tn(g_, a, engine=3), reps=3, warm=1)
+        print(f'gemm_tn k={k} n={nn} engine=3: {ms:7.3f} ms  {2.0 * n * k * nn / ms / 1e9:7.1f} TFLOP/s  {4.0 * n * (k + nn) / ms / 1e6:7.1f} GB/s')
         ga, aa = g_.abs().max().reshape(1), a.abs().max().reshape(1)
         ms3 = timeit(lambda: ops.gemm_tn(g_, a, engine=3, g_amax=ga, a_amax=aa), reps=3, warm=1)
         print(f'     engine 3 with amax supplied: {ms3:7.3f} ms  {4.0 * n * (k + nn) / ms3 / 1e6:7.1f} GB/s')
